@@ -1,4 +1,4 @@
-"""``bench.py --impl reference``: the UNMODIFIED reference (``baseline/_ref``, byte-identical copy of /root/reference,
+"""``bench.py --impl reference``: the UNMODIFIED reference (``oracle/_ref``, byte-identical copy of the original project,
 sha256-checked) running its own stock local-training path on this box.
 
     events "(ip, TRAINING)" -> Coordinator.on_message (reference parser, registry, VirtualWorker per device)
@@ -29,7 +29,8 @@ import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.path.join(HERE, "_ref")
+ORACLE = os.path.join(ROOT, "oracle")
+REF = os.path.join(ORACLE, "_ref")
 SHIMS = os.path.join(HERE, "shims")
 
 PUBLISHED_ROUNDS_PER_S = 0.1133     # BASELINE.md: 12 rounds x 1000 it, 2 x RPi 3B+
@@ -92,14 +93,14 @@ def main(args) -> None:
     if rank != 0:
         return          # the reference's local mode is one process training its workers sequentially
     try:
-        sys.path.insert(0, HERE)
+        sys.path.insert(0, ORACLE)
         import install_ref
         sums = install_ref.verify(REF)
     except Exception as exc:  # noqa: BLE001
-        unavailable(f"baseline/_ref is not installed ({exc}); run `python baseline/install_ref.py` where /root/reference is mounted")
+        unavailable(f"oracle/_ref is not installed ({exc}); run `python oracle/install_ref.py --src <checkout of the original project>`")
         return
     # the reference's flat modules + the stand-ins first on the path; the product's repo root off it
-    sys.path[:] = [REF, SHIMS] + [p for p in sys.path if os.path.abspath(p or ".") not in (ROOT, HERE)]
+    sys.path[:] = [REF, SHIMS] + [p for p in sys.path if os.path.abspath(p or ".") not in (ROOT, HERE, ORACLE)]
 
     import torch
 
@@ -112,7 +113,7 @@ def main(args) -> None:
     real_stdout = sys.stdout
     sys.stdout = sink                      # train_local prints a progress line every 30 batches
     try:
-        import federated_coordinator as fc   # the reference's module (baseline/_ref)
+        import federated_coordinator as fc   # the reference's module (oracle/_ref)
         import settings as ref_settings
         import paho.mqtt.client as mqtt
 
@@ -195,7 +196,7 @@ def main(args) -> None:
                 "timing": "host clock around the same region"},
         "gpu_launches": 0,
         "kernels": "ATen / cuBLAS only (stock torch ops issued by the reference's Python loop)",
-        "reference": {"path": "baseline/_ref", "sha256": sums, "unmodified": True,
+        "reference": {"path": "oracle/_ref", "sha256": sums, "unmodified": True,
                       "entry": "federated_coordinator.Coordinator.on_message -> starting_training_local -> client_federated.train_local",
                       "module_patches": ["federated_coordinator.Timer -> records the callback so the harness can skip the window wait"],
                       "standins": "baseline/shims/{syft,paho}: BUILDER-WRITTEN plain-PyTorch stand-ins for the reference's external, "

@@ -76,7 +76,39 @@ def parse_args():
                     help="after the timed region, run the K rounds once more between two reads of this GPU's NVLink payload counters "
                          "(NVML) and report bytes per round next to the algorithmic count (config.nvlink)")
     ap.add_argument("--no-flush", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed rounds, write what the last timed round returned (global model, per-worker losses) "
+                         "as DIR/<config>_<name>.npy (float32), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config in ("cfg1", "paper", "fulldata", "smpc")):
+        ap.error("--dump-outputs covers the GPU engine configs of --impl ours (ref_local, cfg2, cfg3, ffnn, cfg4, cfg5)")
+    return args
+
+
+DUMP_MAX_ARRAYS = 4                      # the default line dumps two configs x (theta, losses)
+DUMP_MAX_ELEMS = 64 * 1024 * 1024 // 4 // DUMP_MAX_ARRAYS   # 64 MB of float32 in all
+
+
+def dump_outputs(out_dir: str, prefix: str, arrays) -> None:
+    """``out_dir/<prefix>_<name>.npy`` in float32 for every tensor of ``arrays``.  An array of more than
+    ``DUMP_MAX_ELEMS`` elements is stored as a sample: the elements at sorted indices drawn by a generator seeded 0
+    (the same indices every run), flattened."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t is None:
+            continue
+        flat = t.detach().float().cpu().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            arr = flat[idx].numpy()
+        else:
+            arr = t.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), arr)
 
 
 def make_data(model: str, total: int, rank: int, world: int, seed: int = 0):
@@ -389,6 +421,8 @@ def run_engine_config(args, name: str, rank: int, world: int, device, full: bool
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
+    # what the last timed round gave its caller, kept before the untimed passes below move the model on
+    last_outputs = {"theta": engine.global_flat().clone(), "losses": rep.losses}
     dev_ms = max_over_ranks(dev_ms)
     extra = dict(rep.extra)
     # K rounds enqueued in one call: no host in the loop, no flush (what a training of K rounds costs on the device)
@@ -462,6 +496,8 @@ def run_engine_config(args, name: str, rank: int, world: int, device, full: bool
     value = K / (dev_ms * 1e-3)
     if rank != 0:
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, name, last_outputs)
     steps_per_round = epochs * ((n_local + bsz - 1) // bsz)
     cfg = {"name": name, "model": model, "description": desc, "global_batch": bsz * world,
            "batch_size_per_worker": bsz, "seq_len": None, "parallelism": f"fedavg-dp{world}",
@@ -594,7 +630,7 @@ def run_torch_nccl(args, name: str, rank: int, world: int, device):
 def main() -> None:
     args = parse_args()
     if args.impl == "reference":
-        # the unmodified reference from baseline/_ref on its own stock path; nothing of this repo's package is imported
+        # the unmodified reference from oracle/_ref on its own stock path; nothing of this repo's package is imported
         sys.path.insert(0, os.path.join(ROOT, "baseline"))
         import reference_arm
         reference_arm.main(args)

@@ -60,7 +60,7 @@ def worker_id_to_rank(worker_id: str) -> int:
 # transport: an append-only event log and an append-only command log in a key-value store
 # ---------------------------------------------------------------------------------------------------------------------
 class DictStore:
-    """In-process stand-in for the c10d store (``set`` / ``get`` / ``add``): single-process box mode and tests."""
+    """In-process stand-in for the c10d store (``set`` / ``get`` / ``add`` / ``check``): single-process box mode and tests."""
 
     def __init__(self) -> None:
         self._d: Dict[str, bytes] = {}
@@ -83,6 +83,10 @@ class DictStore:
             self._n[key] = self._n.get(key, 0) + int(amount)
             return self._n[key]
 
+    def check(self, keys: List[str]) -> bool:
+        with self._cv:
+            return all(k in self._d for k in keys)
+
 
 class StoreRelay:
     """Two logs on top of a store.  ``post(log, payload)``: ``seq = add(log/n, 1); set(log/seq, payload)``;
@@ -102,9 +106,15 @@ class StoreRelay:
         n = int(self.store.add(f"{self.prefix}/{logname}/n", 0))
         out = []
         for seq in range(self._seen.get(logname, 0) + 1, n + 1):
-            v = self.store.get(f"{self.prefix}/{logname}/{seq}")      # the writer sets it right after taking the number
+            key = f"{self.prefix}/{logname}/{seq}"
+            # the writer sets the entry right after taking its number.  A c10d store client holds its lock while a get
+            # waits for a key, so when the writer is another thread of this process its set would wait for that get:
+            # stop at the first entry not written yet and deliver it on a later poll
+            if not self.store.check([key]):
+                break
+            v = self.store.get(key)
             out.append((seq, v.decode() if isinstance(v, (bytes, bytearray)) else str(v)))
-        self._seen[logname] = max(self._seen.get(logname, 0), n)
+            self._seen[logname] = seq
         return out
 
     def poll(self, logname: str) -> List[str]:

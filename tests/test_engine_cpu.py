@@ -88,6 +88,22 @@ def _serve_commands(relay, control, executed, stop):
         control.command_done(seq)
 
 
+def test_store_relay_poll_does_not_wait_for_an_entry_still_being_written():
+    """A poll that finds a sequence number taken but its entry not yet set returns what precedes it instead of waiting in the
+    store: a c10d store client holds its lock during such a wait, so a writer thread of the same process could not set it."""
+    import datetime
+    import time
+    store = dist.TCPStore("127.0.0.1", 0, 1, True, timeout=datetime.timedelta(seconds=3))
+    writer, reader = StoreRelay(store), StoreRelay(store)
+    writer.post("events", "first")
+    store.add("colearn/box/events/n", 1)                # a second writer has taken number 2 and not set it yet
+    t0 = time.time()
+    assert reader.poll("events") == ["first"] and time.time() - t0 < 1.0
+    store.set("colearn/box/events/2", "second")
+    writer.post("events", "third")
+    assert reader.poll("events") == ["second", "third"] and reader.poll("events") == []
+
+
 def test_box_control_plane_builds_selection_mask():
     """Store log -> in-process bus -> parser / registry / temporal window / selection -> `train` command with the mask."""
     import threading

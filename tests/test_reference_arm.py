@@ -11,10 +11,13 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE = os.path.join(ROOT, "baseline")
-REF = os.path.join(BASE, "_ref")
+ORACLE = os.path.join(ROOT, "oracle")
+REF = os.path.join(ORACLE, "_ref")
+# sha256 of the original project's files, taken from its checkout (tests/golden/reference_sha256.txt)
+GOLDEN_SHA256 = os.path.join(ROOT, "tests", "golden", "reference_sha256.txt")
 
-needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "SHA256SUMS")) and not os.path.exists("/root/reference"),
-                               reason="neither baseline/_ref nor /root/reference is available")
+needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "SHA256SUMS")),
+                               reason="the original project is not installed under oracle/_ref (build() found no checkout of it)")
 
 
 def test_standins_do_not_import_the_product():
@@ -34,18 +37,17 @@ def test_standins_do_not_import_the_product():
 
 @needs_ref
 def test_installed_reference_is_byte_identical():
-    sys.path.insert(0, BASE)
+    sys.path.insert(0, ORACLE)
     try:
         import install_ref
-        if not os.path.exists(os.path.join(REF, "SHA256SUMS")):
-            install_ref.install()
         sums = install_ref.verify(REF)
     finally:
-        sys.path.remove(BASE)
+        sys.path.remove(ORACLE)
     assert {"federated_coordinator.py", "client_federated.py", "datasets.py", "event_parser.py", "settings.py"} <= set(sums)
-    if os.path.exists("/root/reference"):
-        for rel, h in sums.items():
-            assert hashlib.sha256(open(os.path.join("/root/reference", rel), "rb").read()).hexdigest() == h, rel
+    golden = dict(reversed(line.split()) for line in open(GOLDEN_SHA256) if line.strip())
+    assert set(sums) == set(golden)
+    for rel, h in sums.items():
+        assert hashlib.sha256(open(os.path.join(REF, rel), "rb").read()).hexdigest() == h == golden[rel], rel
 
 
 @needs_ref

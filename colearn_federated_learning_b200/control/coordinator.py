@@ -480,8 +480,8 @@ class Coordinator(BusClient):
 def train_virtual_workers(theta: torch.Tensor, model, fed, cfg: FitConfig, round_idx: int):
     """One round of local training for every virtual worker, each starting from ``theta``.
 
-    On a GPU with a persistent-kernel instantiation all K workers train **concurrently in one
-    launch** (one CTA per worker); otherwise they run one after the other through ``local_fit``.
+    On a GPU with a persistent kernel for the model (ops.persistent_path) all K workers train **concurrently in one
+    launch** (one CTA or one cluster per worker); otherwise they run one after the other through ``local_fit``.
     Returns ``(flats[K,P], last_losses[K], sample_counts[K])``.
     """
     k = len(fed.workers)
@@ -490,7 +490,8 @@ def train_virtual_workers(theta: torch.Tensor, model, fed, cfg: FitConfig, round
     counts = [len(fed[w]) for w in fed.workers]
     losses = [0.0] * k
     spec = model.spec if isinstance(model, MLPNet) else None
-    fused = (spec is not None and device.type == "cuda" and ops.net_kind_for(spec.dims, spec.out_activation) is not None)
+    fused = (spec is not None and device.type == "cuda"
+             and ops.persistent_path(spec.dims, spec.out_activation, cfg.batch_size, resolve_loss(cfg.model, cfg.loss), device))
     if fused:
         loss_out = torch.zeros(k, 2, device=device)
         tasks, idx = [], []

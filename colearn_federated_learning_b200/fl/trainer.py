@@ -7,7 +7,8 @@ after ``max_nr_batches`` steps, return the last loss — but on a flat fp32 aren
 small MLP family on a GPU, as ONE persistent-kernel launch (``ops.mlp_local_sgd``).
 
 Three execution paths, chosen by :func:`local_fit`:
-  * ``persistent``  FFNN / MLP / TestingRemote on CUDA → csrc/mlp_persistent.cu
+  * ``persistent``  FFNN / MLP / TestingRemote on CUDA → csrc/mlp_persistent.cu; any other MLP that fits the generic
+                    kernel at batch <= ops.GENERIC_MAX_BATCH → csrc/mlp_generic.cu
   * ``layerwise``   wide MLPs on CUDA → tcgen05 GEMMs + fused loss/SGD kernels (fl/layerwise.py)
   * ``convnet``     ResNet-18 on CUDA → im2col + tcgen05 GEMMs + this repo's BatchNorm / pooling kernels
                     (fl/convnet.py); ``COLEARN_CONV_PATH=torch`` selects the library path instead
@@ -139,7 +140,7 @@ def local_fit(flat: torch.Tensor, model: nn.Module, x: torch.Tensor, y: torch.Te
     if isinstance(model, MLPNet):
         spec = model.spec
         xx = x.view(x.shape[0], -1) if spec.flatten_input else x
-        has_kernel = ops.net_kind_for(spec.dims, spec.out_activation) is not None
+        has_kernel = ops.persistent_path(spec.dims, spec.out_activation, cfg.batch_size, loss, flat.device)
         if not flat.is_cuda or has_kernel:
             last = ops.mlp_local_sgd(flat, spec.dims, xx, y, perm, cfg.batch_size, cfg.lr, cfg.epochs,
                                      cfg.max_nr_batches, loss, spec.out_activation)

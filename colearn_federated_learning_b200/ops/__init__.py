@@ -12,7 +12,7 @@ from . import reference
 from . import _ext
 from . import host  # noqa: F401  (native CPU executor of the MLP local fit)
 from .fused_mlp import (NET_KINDS, LOSS_CODES, net_kind_for, mlp_local_sgd, mlp_local_sgd_multi,  # noqa: F401
-                        mlp_forward, ClientTask, build_client_descs)
+                        mlp_forward, ClientTask, build_client_descs, generic_plan, persistent_path, GENERIC_MAX_BATCH)
 from .reference import make_permutation, total_steps  # noqa: F401
 
 

@@ -24,7 +24,7 @@ EMUL_NAME = "_colearn_emul"     # CPU emulator of the conv kernels (tests on box
 HOST_NAME = "_colearn_host"     # native CPU executor of the MLP local fit (devices / boxes without a GPU)
 SIMT_NAME = "_colearn_simt"     # the persistent-MLP CUDA kernels compiled for the CPU through csrc/host_shim.h (tests)
 
-CU_SOURCES = ["mlp_persistent.cu", "elementwise.cu", "comm.cu", "gemm_tcgen05.cu", "convnet.cu"]
+CU_SOURCES = ["mlp_persistent.cu", "mlp_generic.cu", "elementwise.cu", "comm.cu", "gemm_tcgen05.cu", "convnet.cu"]
 CPP_SOURCES = ["bindings.cpp"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-lineinfo",
@@ -47,7 +47,7 @@ def _stamp(src: str, flags: List[str]) -> str:
     h = hashlib.sha1()
     with open(src, "rb") as f:
         h.update(f.read())
-    for dep in ("colearn_kernels.h", "mlp_v2.inc", "conv_ops.cuh", "conv_bindings.inc"):
+    for dep in ("colearn_kernels.h", "mlp_v2.inc", "conv_ops.cuh", "conv_bindings.inc", "client_desc.inc"):
         with open(os.path.join(CSRC, dep), "rb") as f:
             h.update(f.read())
     h.update(" ".join(flags).encode())
@@ -135,7 +135,7 @@ def simt_path() -> str:
 
 
 def build_simt_emul(force: bool = False) -> str:
-    """g++ build of ``csrc/simt_emul.cpp``: ``mlp_persistent.cu`` + ``mlp_v2.inc`` — the kernel sources themselves —
+    """g++ build of ``csrc/simt_emul.cpp``: ``mlp_persistent.cu`` + ``mlp_v2.inc`` + ``mlp_generic.cu`` — the kernel sources themselves —
     compiled for the CPU with one OS thread per CUDA thread (``csrc/host_shim.h``).  Needs C++20 (``std::barrier``) and
     the CUDA headers, no GPU and no CUDA libraries."""
     ce, cuda_home, inc, flags = _cxx_setup()
@@ -144,9 +144,9 @@ def build_simt_emul(force: bool = False) -> str:
     src = os.path.join(CSRC, "simt_emul.cpp")
     cxx_flags = [f for f in flags if f not in ("-O2", "-std=c++17")] + ["-O1", "-std=c++20", "-pthread", "-Wno-unknown-pragmas",
                                                                         f"-DTORCH_EXTENSION_NAME={SIMT_NAME}"]
-    sources = ["simt_emul.cpp", "simt_mlp.cpp", "simt_elementwise.cpp", "simt_comm.cpp", "simt_convnet.cpp", "simt_gemm.cpp"]
+    sources = ["simt_emul.cpp", "simt_mlp.cpp", "simt_mlp_generic.cpp", "simt_elementwise.cpp", "simt_comm.cpp", "simt_convnet.cpp", "simt_gemm.cpp"]
     h = hashlib.sha1()
-    for dep in sources + ["host_shim.h", "mlp_persistent.cu", "mlp_v2.inc", "elementwise.cu", "comm.cu", "convnet.cu", "gemm_tcgen05.cu", "tcgen05_host_model.h", "conv_bindings.inc", "colearn_kernels.h", "conv_ops.cuh"]:
+    for dep in sources + ["host_shim.h", "mlp_persistent.cu", "mlp_generic.cu", "client_desc.inc", "mlp_v2.inc", "elementwise.cu", "comm.cu", "convnet.cu", "gemm_tcgen05.cu", "tcgen05_host_model.h", "conv_bindings.inc", "colearn_kernels.h", "conv_ops.cuh"]:
         with open(os.path.join(CSRC, dep), "rb") as f:
             h.update(f.read())
     h.update(" ".join(cxx_flags).encode())

@@ -27,32 +27,7 @@ inline T* ptr_of(int64_t p) { return reinterpret_cast<T*>(static_cast<uintptr_t>
 #define CHECK_CUDA_F32(t) TORCH_CHECK((t).is_cuda() && (t).scalar_type() == at::kFloat && (t).is_contiguous(), #t " must be a contiguous CUDA float32 tensor")
 
 // ---- persistent MLP -----------------------------------------------------------------------------
-py::bytes make_client_desc(int64_t x, int64_t y, int64_t perm, int64_t theta_in, int64_t theta_out,
-                           int64_t loss_out, int64_t wait_flag, int64_t wait_value, int64_t signal_flag,
-                           int64_t signal_value, int64_t n, int64_t perm_rows, int64_t y_dim,
-                           double out_scale, int64_t delta_mode, int64_t perm_seed, int64_t perm_row0, int64_t perm_scratch) {
-  ClientDesc d;
-  std::memset(&d, 0, sizeof(d));
-  d.x = ptr_of<const float>(x);
-  d.y = ptr_of<const float>(y);
-  d.perm = ptr_of<const int>(perm);
-  d.theta_in = ptr_of<const float>(theta_in);
-  d.theta_out = ptr_of<float>(theta_out);
-  d.loss_out = ptr_of<float>(loss_out);
-  d.wait_flag = ptr_of<const uint32_t>(wait_flag);
-  d.signal_flag = ptr_of<uint32_t>(signal_flag);
-  d.n = (int)n;
-  d.perm_rows = (int)(perm_rows > 0 ? perm_rows : 1);
-  d.y_dim = (int)y_dim;
-  d.wait_value = (uint32_t)wait_value;
-  d.signal_value = (uint32_t)signal_value;
-  d.out_scale = (float)out_scale;
-  d.delta_mode = (int)delta_mode;
-  d.perm_seed = (uint64_t)perm_seed;
-  d.perm_row0 = (int)perm_row0;
-  d.perm_scratch = ptr_of<int>(perm_scratch);
-  return py::bytes(reinterpret_cast<const char*>(&d), sizeof(d));
-}
+#include "client_desc.inc"
 int64_t client_desc_size() { return (int64_t)sizeof(ClientDesc); }
 
 // p[0:n] *= scale for a raw device pointer (the symmetric work arena)
@@ -82,6 +57,27 @@ void mlp_local_sgd(int64_t net_kind, torch::Tensor descs, int64_t desc_offset, i
 }
 int64_t mlp_net_params(int64_t net_kind) { return mlp_net_num_params((int)net_kind); }
 int64_t mlp_smem_bytes(int64_t net_kind, int64_t batch) { return mlp_local_sgd_smem_bytes((int)net_kind, (int)batch); }
+
+// any small MLP (mlp_generic.cu): one client = one cluster of `cluster` CTAs (0 = the smallest that fits)
+void mlp_local_sgd_generic(std::vector<int64_t> dims, bool sigmoid, torch::Tensor descs, int64_t desc_offset, int64_t n_clients,
+                           int64_t batch_size, int64_t epochs, int64_t max_steps, int64_t loss, double lr, int64_t cluster) {
+  TORCH_CHECK(descs.is_cuda() && descs.scalar_type() == at::kByte && descs.is_contiguous(), "descs must be CUDA uint8");
+  TORCH_CHECK((desc_offset + n_clients) * (int64_t)sizeof(ClientDesc) <= descs.numel(), "descs too small");
+  TORCH_CHECK(dims.size() >= 2 && dims.size() <= 9, "dims: 2..9 widths");
+  std::vector<int> d(dims.begin(), dims.end());
+  c10::cuda::CUDAGuard guard(descs.device());
+  SgdHyper hp;
+  hp.batch_size = (int)batch_size; hp.epochs = (int)epochs; hp.max_steps = (int)max_steps;
+  hp.loss = (int)loss; hp.lr = (float)lr; hp.variant = 0;
+  const ClientDesc* p = reinterpret_cast<const ClientDesc*>(descs.data_ptr<uint8_t>()) + desc_offset;
+  check(launch_mlp_local_sgd_generic(d.data(), (int)d.size() - 1, sigmoid ? 1 : 0, p, (int)n_clients, hp, (int)cluster, cur_stream()),
+        "mlp_local_sgd_generic launch");
+}
+int64_t generic_plan(std::vector<int64_t> dims, int64_t batch_size, int64_t cluster) {
+  if (dims.size() < 2 || dims.size() > 9) return -1;
+  std::vector<int> d(dims.begin(), dims.end());
+  return mlp_generic_plan(d.data(), (int)d.size() - 1, (int)batch_size, (int)cluster, nullptr);
+}
 
 torch::Tensor mlp_forward(int64_t net_kind, torch::Tensor theta, torch::Tensor x, int64_t d_out) {
   CHECK_CUDA_F32(theta); CHECK_CUDA_F32(x);
@@ -580,6 +576,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("mlp_local_sgd", &mlp_local_sgd);
   m.def("mlp_net_params", &mlp_net_params);
   m.def("mlp_smem_bytes", &mlp_smem_bytes);
+  m.def("mlp_local_sgd_generic", &mlp_local_sgd_generic);
+  m.def("mlp_generic_plan", &generic_plan);
   m.def("mlp_forward", &mlp_forward);
   m.def("sgd_step", &sgd_step);
   m.def("fedavg_apply", &fedavg_apply);

@@ -203,6 +203,14 @@ cudaError_t launch_mlp_local_sgd(int net_kind, const ClientDesc* descs, int n_cl
 int mlp_local_sgd_smem_bytes(int net_kind, int batch_size);
 int mlp_net_num_params(int net_kind);
 
+// Persistent local SGD for any small MLP (mlp_generic.cu): layer widths dims[0..L] at run time (L <= 8, dims[L] <= 32, ReLU
+// hidden layers, sigmoid head if `sigmoid`), one client = one thread-block cluster of C in {1, 2, 4, 8} CTAs that splits the
+// weights.  mlp_generic_plan returns the cluster size a launch uses — `cluster` if > 0 and it fits, else the smallest C whose
+// per-CTA footprint fits 227 KB of shared memory — or -1 when none does; *smem_bytes (if non-null) gets its minimum footprint.
+int mlp_generic_plan(const int* dims, int L, int batch_size, int cluster, int* smem_bytes);
+cudaError_t launch_mlp_local_sgd_generic(const int* dims, int L, int sigmoid, const ClientDesc* descs, int n_clients, SgdHyper hp,
+                                         int cluster, cudaStream_t stream);
+
 // Forward-only batched inference/eval for the small nets: out[n, d_out] (post-activation).
 cudaError_t launch_mlp_forward(int net_kind, const float* theta, const float* x, float* out,
                                int n, cudaStream_t stream);

@@ -10,6 +10,8 @@
 //   __shared__        function-local static (blocks run one after the other; contents are as undefined between blocks
 //                     as real shared memory); dynamic shared memory: COLEARN_DYN_SMEM -> a per-block heap buffer
 //   ld.acquire / st.release .sys   __atomic builtins
+//   thread-block cluster   launch_cluster: the blocks of one cluster run concurrently; cluster barrier, peer shared memory and
+//                     the st.async + mbarrier transaction count (mlp_generic.cu) — see the section above launch_cluster
 //   kernel<<<g, b, s, stream>>>(args)   COLEARN_LAUNCH(kernel, g, b, s, stream, args) -> colearn_shim::launch(...)
 //
 // Include this header BEFORE the kernel source and define COLEARN_HOST_SHIM.
@@ -153,6 +155,88 @@ inline void launch(Dim3 grid, Dim3 block, size_t smem_bytes, F&& body) {
       }
     });
   for (auto& th : threads) th.join();
+}
+
+// ---- thread-block clusters (mlp_generic.cu) ------------------------------------------------------------------------------------
+// launch_cluster runs the `cluster` blocks of one cluster CONCURRENTLY (cluster x blockDim OS threads; clusters one after the
+// other), so that blocks can wait for each other.  Distributed shared memory: the same offset in the peer block's `dyn` buffer.
+// mbarrier (transaction-count form): the 8-byte word holds {int32 count, uint32 phase}; count starts at ARRIVE (one pending
+// arrival), expect_tx / complete_tx add and subtract bytes, and the operation that brings it to zero re-arms it and flips the
+// phase (release), which try_wait.parity observes (acquire).
+struct Cluster {
+  std::vector<std::unique_ptr<Block>> blocks;
+  std::unique_ptr<std::barrier<>> bar;
+};
+inline thread_local Cluster* t_cluster = nullptr;
+inline thread_local int t_cluster_rank = 0;
+constexpr int32_t kMbarArrive = 1 << 24;
+
+inline int cluster_rank() { return t_cluster_rank; }
+inline void cluster_sync() { t_cluster->bar->arrive_and_wait(); }
+inline float* dyn_base(Block* b) {
+  uintptr_t p = reinterpret_cast<uintptr_t>(b->dyn.data());
+  return reinterpret_cast<float*>((p + 15) & ~(uintptr_t)15);
+}
+template <class T>
+inline T* peer_ptr(T* local, int peer) {
+  const ptrdiff_t off = reinterpret_cast<char*>(local) - reinterpret_cast<char*>(dyn_smem());
+  return reinterpret_cast<T*>(reinterpret_cast<char*>(dyn_base(t_cluster->blocks[(size_t)peer].get())) + off);
+}
+inline void mbar_init(uint64_t* bar) {
+  int32_t* w = reinterpret_cast<int32_t*>(bar);
+  __atomic_store_n(w, kMbarArrive, __ATOMIC_RELAXED);
+  __atomic_store_n(reinterpret_cast<uint32_t*>(w + 1), 0u, __ATOMIC_RELEASE);
+}
+inline void mbar_add(uint64_t* bar, int32_t delta) {
+  int32_t* w = reinterpret_cast<int32_t*>(bar);
+  if (__atomic_add_fetch(w, delta, __ATOMIC_SEQ_CST) == 0) {
+    __atomic_store_n(w, kMbarArrive, __ATOMIC_RELAXED);
+    __atomic_fetch_xor(reinterpret_cast<uint32_t*>(w + 1), 1u, __ATOMIC_RELEASE);
+  }
+}
+// st.async of one float into the peer's copy of `local` + complete_tx(4) on the peer's copy of `bar`
+inline void push_to_peer(float* local, float v, int peer, uint64_t* bar) {
+  *peer_ptr(local, peer) = v;
+  mbar_add(peer_ptr(bar, peer), -4);
+}
+inline void mbar_wait(uint64_t* bar, uint32_t parity, uint32_t bytes, bool arrive) {
+  if (arrive) mbar_add(bar, (int32_t)bytes - kMbarArrive);
+  const uint32_t* phase = reinterpret_cast<const uint32_t*>(bar) + 1;
+  while ((__atomic_load_n(phase, __ATOMIC_ACQUIRE) & 1u) == (parity & 1u)) std::this_thread::yield();
+}
+
+template <class F>
+inline void launch_cluster(Dim3 grid, unsigned cluster, Dim3 block, size_t smem_bytes, F&& body) {
+  const unsigned nthreads = block.count();
+  if (nthreads == 0 || grid.x == 0 || cluster == 0) return;
+  for (unsigned c0 = 0; c0 < grid.x; c0 += cluster) {
+    Cluster cl;
+    for (unsigned r = 0; r < cluster; ++r) {
+      cl.blocks.emplace_back(std::make_unique<Block>((int)nthreads, smem_bytes));
+      Block& b = *cl.blocks.back();
+      b.block_idx = Dim3{c0 + r};
+      b.block_dim = block;
+      b.grid_dim = grid;
+    }
+    cl.bar = std::make_unique<std::barrier<>>((std::ptrdiff_t)(nthreads * cluster));
+    std::vector<std::thread> threads;
+    threads.reserve(nthreads * cluster);
+    for (unsigned r = 0; r < cluster; ++r)
+      for (unsigned t = 0; t < nthreads; ++t)
+        threads.emplace_back([&, r, t] {
+          t_linear = t;
+          t_threadIdx = Dim3{t % block.x, (t / block.x) % block.y, t / (block.x * block.y)};
+          t_block = cl.blocks[r].get();
+          t_cluster = &cl;
+          t_cluster_rank = (int)r;
+          body();
+          t_block->bar.arrive_and_drop();
+          t_block->warp_bar[t / 32]->arrive_and_drop();
+          cl.bar->arrive_and_drop();
+          t_cluster = nullptr;
+        });
+    for (auto& th : threads) th.join();
+  }
 }
 
 }  // namespace colearn_shim

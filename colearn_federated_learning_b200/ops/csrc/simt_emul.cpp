@@ -7,6 +7,8 @@
 
 #include "colearn_kernels.h"
 
+#include <cstring>
+
 namespace py = pybind11;
 
 namespace {
@@ -78,6 +80,28 @@ Tensor mlp_local_sgd(int64_t net_kind, Tensor theta_in, std::vector<Tensor> thet
   }
   return losses;
 }
+
+// mlp_generic.cu: descs is a CPU uint8 tensor of ClientDescs packed by make_client_desc from host pointers; the clusters run one
+// after the other, the CTAs of a cluster concurrently.  Same arguments as the CUDA binding.
+void mlp_local_sgd_generic(std::vector<int64_t> dims, bool sigmoid, Tensor descs, int64_t desc_offset, int64_t n_clients, int64_t batch_size,
+                           int64_t epochs, int64_t max_steps, int64_t loss, double lr, int64_t cluster) {
+  TORCH_CHECK(!descs.is_cuda() && descs.scalar_type() == at::kByte && descs.is_contiguous(), "descs must be CPU uint8");
+  TORCH_CHECK((desc_offset + n_clients) * (int64_t)sizeof(colearn::ClientDesc) <= descs.numel(), "descs too small");
+  TORCH_CHECK(dims.size() >= 2 && dims.size() <= 9, "dims: 2..9 widths");
+  std::vector<int> d(dims.begin(), dims.end());
+  colearn::SgdHyper hp;
+  hp.batch_size = (int)batch_size; hp.epochs = (int)epochs; hp.max_steps = (int)max_steps;
+  hp.loss = (int)loss; hp.lr = (float)lr; hp.variant = 0;
+  const colearn::ClientDesc* p = reinterpret_cast<const colearn::ClientDesc*>(descs.data_ptr<uint8_t>()) + desc_offset;
+  py::gil_scoped_release nogil;
+  TORCH_CHECK(cudaSuccess == colearn::launch_mlp_local_sgd_generic(d.data(), (int)d.size() - 1, sigmoid ? 1 : 0, p, (int)n_clients, hp, (int)cluster, nullptr), "launch_mlp_local_sgd_generic (host shim) failed");
+}
+int64_t mlp_generic_plan(std::vector<int64_t> dims, int64_t batch_size, int64_t cluster) {
+  if (dims.size() < 2 || dims.size() > 9) return -1;
+  std::vector<int> d(dims.begin(), dims.end());
+  return colearn::mlp_generic_plan(d.data(), (int)d.size() - 1, (int)batch_size, (int)cluster, nullptr);
+}
+#include "client_desc.inc"
 
 Tensor mlp_forward(int64_t net_kind, Tensor theta, Tensor x, int64_t d_out) {
   TORCH_CHECK(x.dim() == 2, "x [n, d_in]");
@@ -382,6 +406,9 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         py::arg("batch_size"), py::arg("epochs"), py::arg("max_steps"), py::arg("loss"), py::arg("lr"), py::arg("variant"), py::arg("out_scales"),
         py::arg("delta_mode"), py::arg("flags"), py::arg("perm_seed") = 0, py::arg("perm_row0") = 0, py::arg("perm_scratch") = py::none());
   m.def("mlp_forward", &mlp_forward);
+  m.def("mlp_local_sgd_generic", &mlp_local_sgd_generic);
+  m.def("mlp_generic_plan", &mlp_generic_plan);
+  m.def("make_client_desc", &make_client_desc);
   m.def("mlp_net_params", [](int64_t kind) { return (int64_t)colearn::mlp_net_num_params((int)kind); });
   m.def("sgd_step", &sgd_step);
   m.def("fedavg_apply", &fedavg_apply);

@@ -4,8 +4,9 @@ One launch runs the *entire* local fit of one or many federated clients (one CTA
 reference's per-batch ``zero_grad → forward → loss → backward → step`` loop
 (``client_federated.py:101-120`` locally; PySyft ``_fit`` remotely, SURVEY C27) never returns to
 the host.  Supported architectures are the compile-time instantiations FFNN (10-50-30-10-1,
-sigmoid), MLP (10-64-64-2) and TestingRemote (2-50-10-1); anything else goes through the
-layer-wise trainer (``fl/layerwise.py``).
+sigmoid), MLP (10-64-64-2) and TestingRemote (2-50-10-1).  Every other MLP with at most 8 layers and a head of at
+most 32 outputs runs the run-time-shaped kernel of ``csrc/mlp_generic.cu`` (one client = one thread-block cluster that
+splits the weights); callers prefer it to the layer-wise trainer (``fl/layerwise.py``) up to ``GENERIC_MAX_BATCH``.
 """
 from __future__ import annotations
 
@@ -40,11 +41,43 @@ def resolve_variant(kind: int, variant: Optional[int] = None) -> int:
     return BEST_VARIANT.get(kind, 5) if v == 0 else v
 
 
+# Largest batch at which the callers (fl/trainer.local_fit, the engine's star round, train_virtual_workers) prefer the generic
+# kernel to the layer-wise tcgen05 trainer for an MLP without a specialised kernel.  profiles/README.md R3.1 has the measured
+# crossover; the cap stays at 8 so that larger batches keep the layer-wise / two-shot paths they take today.
+GENERIC_MAX_BATCH = 8
+GENERIC_MAX_LAYERS = 8
+GENERIC_MAX_DOUT = 32
+
 PtrLike = Union[torch.Tensor, int, None]
 
 
 def net_kind_for(dims: Sequence[int], out_activation: str = "none") -> Optional[int]:
     return NET_KINDS.get((tuple(int(d) for d in dims), out_activation))
+
+
+def generic_plan(dims: Sequence[int], out_activation: str, batch_size: int, cluster: int = 0,
+                 loss: Optional[str] = None) -> Optional[int]:
+    """Cluster size (CTAs per client) the generic kernel uses for this MLP, or None when it cannot train it: a head wider
+    than 32, more than 8 layers, an output activation other than none / sigmoid, ``bce`` without a sigmoid head, or weights
+    that do not fit the shared memory of 8 CTAs.  ``cluster`` > 0 asks for that size (None if it is not legal or does not
+    fit)."""
+    dims = [int(d) for d in dims]
+    if len(dims) < 2 or len(dims) - 1 > GENERIC_MAX_LAYERS or dims[-1] > GENERIC_MAX_DOUT or min(dims) < 1:
+        return None
+    if out_activation not in ("none", "sigmoid") or (loss == "bce" and out_activation != "sigmoid"):
+        return None
+    c = int(_ext.require().mlp_generic_plan(dims, max(1, int(batch_size)), int(cluster)))
+    return c if c > 0 else None
+
+
+def persistent_path(dims: Sequence[int], out_activation: str, batch_size: int, loss: Optional[str] = None, device=None) -> bool:
+    """True when a whole local fit of this MLP is one persistent-kernel launch on ``device``: a specialised kernel
+    (NET_KINDS), or — on a CUDA device, up to GENERIC_MAX_BATCH — the generic one."""
+    if net_kind_for(dims, out_activation) is not None:
+        return True
+    if device is not None and torch.device(device).type != "cuda":
+        return False
+    return int(batch_size) <= GENERIC_MAX_BATCH and generic_plan(dims, out_activation, batch_size, loss=loss) is not None
 
 
 def _ptr(t: PtrLike) -> int:
@@ -110,13 +143,23 @@ def _prep_xy(x: torch.Tensor, y: torch.Tensor, loss: str) -> Tuple[torch.Tensor,
 
 def mlp_local_sgd_multi(dims: Sequence[int], out_activation: str, descs: torch.Tensor, n_clients: int,
                         batch_size: int = 1, lr: float = 0.01, epochs: int = 1, max_nr_batches: int = -1,
-                        loss: str = "xent", desc_offset: int = 0, variant: Optional[int] = None) -> None:
-    """Launch ``n_clients`` CTAs from a packed descriptor tensor (see :func:`build_client_descs`)."""
+                        loss: str = "xent", desc_offset: int = 0, variant: Optional[int] = None, cluster: int = 0) -> None:
+    """Launch ``n_clients`` clients from a packed descriptor tensor (see :func:`build_client_descs`): one CTA each for the
+    specialised networks, one cluster each for any other MLP (``cluster`` forces its size; tests)."""
     kind = net_kind_for(dims, out_activation)
-    if kind is None:
-        raise ValueError(f"no persistent-kernel instantiation for dims={tuple(dims)} act={out_activation}")
     if loss == "bce" and out_activation != "sigmoid":
         raise ValueError("bce needs a sigmoid head")
+    if kind is None:
+        c = generic_plan(dims, out_activation, batch_size, cluster, loss)
+        if c is None:
+            raise ValueError(f"no persistent kernel for dims={tuple(dims)} act={out_activation} batch={batch_size} "
+                             f"cluster={cluster}: the generic kernel takes <= {GENERIC_MAX_LAYERS} layers, a head of "
+                             f"<= {GENERIC_MAX_DOUT} and weights that fit 8 CTAs")
+        _ext.require().mlp_local_sgd_generic([int(d) for d in dims], out_activation == "sigmoid", descs, int(desc_offset),
+                                             int(n_clients), int(batch_size), int(epochs),
+                                             int(max_nr_batches if max_nr_batches is not None else -1), LOSS_CODES[loss],
+                                             float(lr), c)
+        return
     _ext.require().mlp_local_sgd(kind, descs, int(desc_offset), int(n_clients), int(batch_size), int(epochs),
                                  int(max_nr_batches if max_nr_batches is not None else -1), LOSS_CODES[loss], float(lr),
                                  resolve_variant(kind, variant))
@@ -125,7 +168,7 @@ def mlp_local_sgd_multi(dims: Sequence[int], out_activation: str, descs: torch.T
 def mlp_local_sgd(flat: torch.Tensor, dims: Sequence[int], x: torch.Tensor, y: torch.Tensor,
                   perm: Optional[torch.Tensor], batch_size: int = 1, lr: float = 0.01, epochs: int = 1,
                   max_nr_batches: int = -1, loss: str = "xent", out_activation: str = "none",
-                  return_mean: bool = False, variant: Optional[int] = None) -> torch.Tensor:
+                  return_mean: bool = False, variant: Optional[int] = None, cluster: int = 0) -> torch.Tensor:
     """Single-client in-place local SGD on ``flat``; returns the last batch loss (0-dim tensor).
 
     CPU tensors run ``reference.mlp_local_sgd`` (identical semantics); CUDA tensors run the
@@ -147,7 +190,8 @@ def mlp_local_sgd(flat: torch.Tensor, dims: Sequence[int], x: torch.Tensor, y: t
         perm = perm.to(flat.device, torch.int32).contiguous()
     task = ClientTask(x=x, y=y, theta_in=flat, theta_out=flat, perm=perm, loss_out=loss_out)
     descs = build_client_descs([task], flat.device)
-    mlp_local_sgd_multi(dims, out_activation, descs, 1, batch_size, lr, epochs, max_nr_batches, loss, variant=variant)
+    mlp_local_sgd_multi(dims, out_activation, descs, 1, batch_size, lr, epochs, max_nr_batches, loss, variant=variant,
+                        cluster=cluster)
     return loss_out[1 if return_mean else 0]
 
 

@@ -95,7 +95,9 @@ class FederatedEngine:
         self.weighted = weighted
         self.server_lr = server_lr
         self.seed = seed
-        persistent = self.spec is not None and ops.net_kind_for(self.spec.dims, self.spec.out_activation) is not None
+        # a specialised persistent kernel, or (CUDA, batch <= ops.GENERIC_MAX_BATCH) the generic one
+        persistent = self.spec is not None and ops.persistent_path(self.spec.dims, self.spec.out_activation, batch_size,
+                                                                   self.cfg.loss, self.device)
         if algo == "auto":
             algo = "star" if persistent else "twoshot"
         if algo == "star" and backend == "fused" and not persistent:
